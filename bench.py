@@ -2,6 +2,7 @@
 dominant kernel and the reference's CPU path timed beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|northstar]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload = "cfg2", BASELINE.json configs[1]): synthetic 480p (854x480 -> 864x480 padded, 30x54 = 1620
@@ -231,9 +232,11 @@ def run_ours(args, wl, rank, world, dev):
         torch.cuda.synchronize(dev)
 
     state = {'t': 1}
+    res = {}
 
-    def device_arm(steps, lookahead, profile):
-        """`steps` frames with inputs resident in HBM; returns (per-step event marks, host enqueue ms/step)."""
+    def device_arm(steps, lookahead, profile, keep_last=False):
+        """`steps` frames with inputs resident in HBM; returns (per-step event marks, host enqueue ms/step).  keep_last:
+        a copy of the last step's output (taken after the last mark) goes to res['outputs']."""
         t = state['t']
         marks = [torch.cuda.Event(enable_timing=True) for _ in range(steps + 1)]
         if profile:
@@ -242,13 +245,15 @@ def run_ours(args, wl, rank, world, dev):
         h0 = time.perf_counter()
         for j in range(steps):
             if lookahead:
-                proc.step(frames_dev[t], next_image=frames_dev[t + 1] if j + 1 < steps else None)
+                prob = proc.step(frames_dev[t], next_image=frames_dev[t + 1] if j + 1 < steps else None)
             else:
-                proc.step(frames_dev[t])
+                prob = proc.step(frames_dev[t])
             marks[j + 1].record()
             t += 1
         host_ms = (time.perf_counter() - h0) * 1e3 / steps
         state['t'] = t
+        if keep_last:
+            res['outputs'] = {'prob': prob.clone()}       # a CUDA-graph replay returns a buffer the next step overwrites
         return marks, host_ms
 
     def e2e_arm(steps, lookahead):
@@ -294,7 +299,6 @@ def run_ours(args, wl, rank, world, dev):
         state['t'] = t0 + steps
         return e0, e1, host_ms
 
-    res = {}
     with torch.inference_mode():
         for _ in range(warm):
             proc.step(frames_dev[state['t']])
@@ -307,7 +311,7 @@ def run_ours(args, wl, rank, world, dev):
         launches0 = K_.LAUNCH_COUNT
         if args.phase_timing:
             K_.phase_timing(True)
-        marks, host_dev = device_arm(K, False, True)
+        marks, host_dev = device_arm(K, False, True, keep_last=bool(args.dump_outputs))
         barrier()
         stop.set(); th.join()
         launches = K_.LAUNCH_COUNT - launches0
@@ -415,6 +419,18 @@ def run_ours(args, wl, rank, world, dev):
             traceback.print_exc()
             res['parity'] = {'error': f'{type(e).__name__}: {e}'[:300]}
     return res
+
+
+def dump_outputs(out_dir, outputs):
+    """What the headline arm's last timed step returned to its caller -- InferenceCore.step's per-object probabilities
+    [1 + objects, H, W] -- as float32 .npy files, for comparing two builds output for output on the same seeded inputs."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.detach().float().cpu().numpy()
+        assert a.nbytes <= 64 * 2**20, (name, a.shape)
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+        log(f'[dump] {name}: {a.shape} float32 -> {out_dir}')
 
 
 def parity_check(proc, cfg, frame, dev):
@@ -752,6 +768,8 @@ def main():
     ap.add_argument('--no-sharded-read', action='store_true', help='skip the key-sharded read benchmark at N > 1')
     ap.add_argument('--no-northstar', action='store_true', help='skip the north-star-size memory-read micro-benchmark')
     ap.add_argument('--cpu-seconds', type=float, default=150.0)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the last timed step\'s outputs (InferenceCore.step probabilities) as DIR/<name>.npy')
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -775,6 +793,8 @@ def main():
     if world > 1:
         torch.distributed.init_process_group('nccl', device_id=dev)
     res = run_ours(args, wl, rank, world, dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res.pop('outputs'))
     conv_roof = None
     if rank == 0 and not args.no_northstar:
         try:

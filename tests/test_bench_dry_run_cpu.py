@@ -47,3 +47,22 @@ def test_bench_drop_in_only_and_no_checks():
     line, err = _run('--no-lookahead', '--no-cpu-baseline', '--no-parity-check')
     assert line['with_encoder_lookahead'] is None and line['cpu_baseline'] is None and line['parity_check'] is None
     assert line['value'] > 0 and line['e2e']['value'] > 0
+
+
+def test_bench_dumps_the_last_timed_step_and_repeats_it(tmp_path):
+    """--dump-outputs: the probabilities InferenceCore.step returned in the last timed step, float32, the same from run to
+    run with the same arguments (seeded inputs); --steps sets the number of timed steps."""
+    import numpy as np
+    outs = []
+    for run, steps in (('a', 5), ('b', 5), ('c', 4)):
+        d = tmp_path / run
+        line, err = _run('--no-lookahead', '--no-cpu-baseline', '--no-parity-check', '--steps', str(steps),
+                         '--dump-outputs', str(d))
+        assert line['steps'] == steps and line['latency_ms']['frames'] == steps
+        assert sorted(os.listdir(d)) == ['prob.npy']
+        outs.append(np.load(d / 'prob.npy'))
+    a, b, c = outs
+    assert a.dtype == np.float32 and a.ndim == 3 and a.shape[0] == 1 + line['config']['objects']
+    assert np.isfinite(a).all() and np.allclose(a.sum(0), 1, atol=1e-4)
+    assert np.array_equal(a, b)
+    assert not np.array_equal(a, c)             # one timed step fewer: another frame's output

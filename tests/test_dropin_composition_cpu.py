@@ -1,16 +1,31 @@
 """`cutie/` (this repo's drop-in shim) composed with a reference checkout on sys.path: modules the shim provides -- the
 hot-path surface -- win; everything else (dataset readers, palette, ...) resolves to the reference's own files, so
-eval_vos.py-style imports work unchanged with this repo placed AHEAD of the reference on PYTHONPATH.  Needs the
-read-only reference checkout of the build container (skipped elsewhere)."""
+eval_vos.py-style imports work unchanged with this repo placed AHEAD of the reference on PYTHONPATH.  The reference
+checkout is a stand-in with the reference's package layout (hkchengrex/Cutie: `cutie/` without an __init__.py, empty
+sub-package __init__.py files) and one-line modules at the paths involved."""
 import os
 import subprocess
 import sys
 
-import pytest
-
 from tests.conftest import ROOT
 
-REF = '/root/reference'
+# modules of the reference that the shim also provides, and modules only the reference has
+SHIM_PROVIDED = ['cutie/inference/inference_core.py', 'cutie/inference/memory_manager.py',
+                 'cutie/inference/kv_memory_store.py', 'cutie/inference/object_manager.py', 'cutie/model/cutie.py',
+                 'cutie/utils/get_default_model.py']
+REFERENCE_ONLY = ['cutie/inference/data/video_reader.py', 'cutie/inference/data/vos_test_dataset.py',
+                  'cutie/utils/palette.py']
+
+
+def _stand_in_reference(root):
+    for pkg in ('cutie/inference', 'cutie/inference/data', 'cutie/model', 'cutie/utils'):
+        os.makedirs(os.path.join(root, pkg), exist_ok=True)
+        open(os.path.join(root, pkg, '__init__.py'), 'w').close()
+    for f in SHIM_PROVIDED + REFERENCE_ONLY:
+        with open(os.path.join(root, f), 'w') as fh:
+            fh.write('"""stand-in for the reference module at this path"""\n')
+    return root
+
 
 PROBE = r'''
 import importlib, json
@@ -25,9 +40,9 @@ print(json.dumps(out))
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'cutie')), reason='reference checkout not present')
 def test_shim_wins_for_the_hot_path_and_defers_to_the_reference_elsewhere(tmp_path):
     import json
+    REF = _stand_in_reference(str(tmp_path / 'reference'))
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([ROOT, REF]))
     r = subprocess.run([sys.executable, '-c', PROBE], capture_output=True, text=True, cwd=str(tmp_path), env=env, timeout=300)
     assert r.returncode == 0, r.stderr[-2000:]
