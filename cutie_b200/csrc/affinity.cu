@@ -12,8 +12,6 @@
 //   the winners, optional fixed-point usage accumulation (deterministic).
 // Kernel 3  readout_gather_kernel  one warp per query x object: gathers the k winning 1 KB value rows,
 //   accumulates in registers, transposes through smem to the channel-major [B,K,CV,Q] output.
-#include <stdlib.h>
-
 #include "topk_common.cuh"
 #include "affinity_internal.cuh"
 
@@ -32,7 +30,6 @@ struct ScanParams {
   const float* qe;
   long long Q;
   long long n_total;
-  long long samp_begin, samp_stride, samp_count;   // virtual index i -> token samp_begin + i*samp_stride
   int top_k;
   int kpad;
   int tiles_per_split;
@@ -62,9 +59,8 @@ __device__ __forceinline__ void load_key_tile(ScanSmem& sm, int stage, const Sca
     long long i = i0 + r;
     float* dst = &sm.ks[stage][r][4 * c4];
     if (i < i_end) {
-      const long long g = p.samp_begin + i * p.samp_stride;
-      int s = seg_of(p.segs.begin, p.segs.nseg, g);
-      const float* src = p.segs.key[s] + (long long)b * p.segs.key_bs[s] + (g - p.segs.begin[s]) * CKD + 4 * c4;
+      int s = seg_of(p.segs.begin, p.segs.nseg, i);
+      const float* src = p.segs.key[s] + (long long)b * p.segs.key_bs[s] + (i - p.segs.begin[s]) * CKD + 4 * c4;
       cp_async16(dst, src);
     } else {
       *reinterpret_cast<float4*>(dst) = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -73,9 +69,8 @@ __device__ __forceinline__ void load_key_tile(ScanSmem& sm, int stage, const Sca
   if (tid < TK) {
     long long i = i0 + tid;
     if (i < i_end) {
-      const long long g = p.samp_begin + i * p.samp_stride;
-      int s = seg_of(p.segs.begin, p.segs.nseg, g);
-      cp_async4(&sm.sh[stage][tid], p.segs.shr[s] + (long long)b * p.segs.shr_bs[s] + (g - p.segs.begin[s]));
+      int s = seg_of(p.segs.begin, p.segs.nseg, i);
+      cp_async4(&sm.sh[stage][tid], p.segs.shr[s] + (long long)b * p.segs.shr_bs[s] + (i - p.segs.begin[s]));
     } else {
       sm.sh[stage][tid] = 0.f;
     }
@@ -91,7 +86,7 @@ __global__ void __launch_bounds__(NT, 1) affinity_scan_kernel(const ScanParams p
   const long long q0 = (long long)blockIdx.x * TQ;
   const long long split_begin = (long long)split * p.tiles_per_split * TK;
   long long split_end = split_begin + (long long)p.tiles_per_split * TK;
-  if (split_end > p.samp_count) split_end = p.samp_count;
+  if (split_end > p.n_total) split_end = p.n_total;
   const int ntiles = split_end > split_begin ? (int)((split_end - split_begin + TK - 1) / TK) : 0;
   const float scale = rsqrtf((float)CKD);
 
@@ -198,7 +193,7 @@ __global__ void __launch_bounds__(NT, 1) affinity_scan_kernel(const ScanParams p
         const unsigned long long ce = __shfl_sync(0xffffffffu, ent, src);
         const float s = __uint_as_float((unsigned)(ce >> 32));
         const int ql = (int)((ce >> 24) & 0xffu);
-        const int idx = (int)(p.samp_begin + (split_begin + (long long)(ce & 0xffffffu)) * p.samp_stride);
+        const int idx = (int)(split_begin + (long long)(ce & 0xffffffu));
         const float kth = sm.lval[ql][p.top_k - 1];
         if (s > kth || (s == kth && idx < sm.lidx[ql][p.top_k - 1])) {
           float tau = list_insert<NS>(&sm.lval[ql][0], &sm.lidx[ql][0], lane, p.top_k, s, idx);
@@ -373,69 +368,40 @@ static int pick_splits(long long B, long long Q, long long count) {
 }
 
 // ---- plan: which passes run for a bank of n_total tokens ------------------------------------------------
-// exact  (levels == 0): n_total < tc_min                 exact fp32 scan of everything (affinity_scan_kernel)
-// filter (levels >= 1): nested strided samples, coarsest first (strides ... 256, 16, 1).  The coarsest sample has
-//                       <= TC_CAP tokens so every one of them is a candidate; each level hands an upper bound of its
-//                       k-th smallest energy to the next; the last level (stride 1) is re-ranked exactly.
-struct Plan {
-  int levels;             // 0 = exact scan only
-  long long stride[8];    // coarsest first, last == 1
-};
-constexpr int TC_CAP = 4096;           // candidate slots per query (also the largest all-pass coarsest sample)
-constexpr int TC_CAP_BIG = 16384;      // slots per query used for the candidate lists (overflow => exhaustive rescan of that query)
+// exact  (0): n_total < tc_min or n_total < 2 top_k, or a call without key images: exact fp32 scan of everything
+//             (affinity_scan_kernel + topk_merge_kernel)
+// filter (1): the FP16 plan over the key images (affinity_f16.cu): threshold sample pass, threshold select, candidate
+//             filter over the whole bank, exact re-rank of the survivors
+constexpr int CAND_CAP = 16384;        // candidate slots per query (overflow => exhaustive rescan of that query)
 
 static long long g_tc_min_override = -1;
-static long long g_image_level_launches = 0;     // filter levels served from a key image (tests / diagnostics)
+static long long g_image_level_launches = 0;     // filter passes served from a key image (tests / diagnostics)
 
-static long long tc_min_tokens() {
-  if (g_tc_min_override >= 0) return g_tc_min_override;
-  static long long v = -1;
-  if (v < 0) {
-    const char* e = getenv("CUTIE_B200_TC_MIN");
-    v = e ? atoll(e) : 6144;
-    const char* off = getenv("CUTIE_B200_NO_TC");
-    if (off && off[0] == '1') v = (1ll << 40);
-  }
-  return v;
-}
+static long long tc_min_tokens() { return g_tc_min_override >= 0 ? g_tc_min_override : 6144; }
 
-static Plan make_plan(long long n_total, int top_k) {
-  Plan pl;
-  pl.levels = 0;
-  if (n_total < tc_min_tokens() || n_total < 2 * (long long)top_k) return pl;
-  long long st[8];
-  int n = 0;
-  st[n++] = 1;
-  while ((n_total + st[n - 1] - 1) / st[n - 1] > TC_CAP && n < 8) { st[n] = st[n - 1] * 16; ++n; }
-  // the coarsest sample must still hold at least 2k tokens to give a meaningful bound
-  while (n > 1 && (n_total + st[n - 1] - 1) / st[n - 1] < 2 * (long long)top_k) --n;
-  if ((n_total + st[n - 1] - 1) / st[n - 1] > TC_CAP) return pl;      // cannot seed the thresholds: exact scan
-  pl.levels = n;
-  for (int i = 0; i < n; ++i) pl.stride[i] = st[n - 1 - i];
-  return pl;
+static bool filter_plan(long long n_total, int top_k) {
+  return n_total >= tc_min_tokens() && n_total >= 2 * (long long)top_k;
 }
 
 struct WsLayout {
-  size_t part, cand_idx, cand_e, count, dmax, emax0, emax1;   // byte offsets
+  size_t part, cand_idx, cand_e, count, emax;   // byte offsets
   size_t total;
 };
 
+// Every call can take the exact scan (a call without key images always does); banks that qualify for the filter plan
+// also get its buffers.
 static WsLayout ws_layout(long long B, long long Q, long long n_total, int top_k) {
   const int kpad = top_k <= 32 ? 32 : 64;
-  const Plan pl = make_plan(n_total, top_k);
   WsLayout w;
   memset(&w, 0, sizeof(w));
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-  if (pl.levels == 0) {
-    w.part = take((size_t)B * pick_splits(B, Q, n_total) * Q * kpad * 8);
-  } else {
-    w.cand_idx = take((size_t)B * Q * TC_CAP_BIG * 4);
-    w.cand_e = take((size_t)B * Q * TC_CAP_BIG * 4);
+  w.part = take((size_t)B * pick_splits(B, Q, n_total) * Q * kpad * 8);
+  if (filter_plan(n_total, top_k)) {
+    w.cand_idx = take((size_t)B * Q * CAND_CAP * 4);
+    w.cand_e = take((size_t)B * Q * CAND_CAP * 4);
     w.count = take((size_t)B * Q * 4);
-    w.dmax = take((size_t)B * Q * 4);
-    w.emax0 = take((size_t)B * Q * 4);
-    w.emax1 = take((size_t)B * Q * 4);
+    w.emax = take((size_t)B * Q * 4);
   }
   w.total = off + 256;
   return w;
@@ -444,7 +410,7 @@ static WsLayout ws_layout(long long B, long long Q, long long n_total, int top_k
 static int run_exact(const ScanParams& base, long long B, int nsplit, int* out_idx, float* out_w, float* out_sim,
                      unsigned long long* usage_acc, cudaStream_t st) {
   ScanParams sp = base;
-  const long long ntiles = (sp.samp_count + TK - 1) / TK;
+  const long long ntiles = (sp.n_total + TK - 1) / TK;
   sp.nsplit = nsplit;
   sp.tiles_per_split = (int)((ntiles + nsplit - 1) / nsplit);
   if ((long long)sp.tiles_per_split * TK >= (1ll << 24)) return fail(-1, "%s: split too long", "run_exact");
@@ -509,71 +475,14 @@ static int phase_begin(cudaStream_t st) {
   return slot;
 }
 
-// Optional precomputed operand images of the arenas the segments live in (cutie_bank_key_image).
+// Precomputed operand images of the arenas the segments live in (cutie_bank_key_image).
 struct ImageArgs {
-  bool on;
   const float* mu;            // [B][64] key centre of the images (null = 0)
   const int* seed_idx;        // [B][Q][kpad] threshold seeds (null = none)
   const float* img[kMaxSeg];
   long long bs[kMaxSeg];      // batch stride (floats)
   long long phys[kMaxSeg];    // physical index of the segment's first token inside its arena
 };
-
-// One filter level: zero the per-query counters, tcgen05 filter over the stride-`stride` sample.
-static int run_filter_level(const ScanParams& base, long long B, long long stride, const float* emax_in, char* ws,
-                            const WsLayout& wl, float* dbg_energy, const ImageArgs& ia, cudaStream_t st) {
-  TcFilterParams fp;
-  memset(&fp, 0, sizeof(fp));
-  fp.segs = base.segs;
-  fp.qk = base.qk;
-  fp.qe = base.qe;
-  fp.Q = base.Q;
-  fp.samp_begin = 0;
-  fp.samp_stride = stride;
-  fp.samp_count = (base.n_total + stride - 1) / stride;
-  fp.nsplit = tc_split_count(B, base.Q, fp.samp_count);
-  const long long ntiles = (fp.samp_count + 127) / 128;
-  fp.tiles_per_split = (int)((ntiles + fp.nsplit - 1) / fp.nsplit);
-  fp.emax_in = emax_in;
-  fp.cand_idx = (int*)(ws + wl.cand_idx);
-  fp.cand_e = (float*)(ws + wl.cand_e);
-  fp.count = (int*)(ws + wl.count);
-  fp.dmax = (float*)(ws + wl.dmax);
-  fp.cap = TC_CAP_BIG;
-  fp.dbg_energy = dbg_energy;
-  if (ia.on && stride == 1 && emax_in != nullptr) {
-    // the whole bank, one bulk copy per physical 128-token tile of each segment's arena
-    fp.use_img = 1;
-    static int chunks = -1, prefetch = -1;
-    if (chunks < 0) {
-      const char* e = getenv("CUTIE_B200_IMG_CHUNKS");
-      chunks = e ? atoi(e) : 1;        // measured at cfg 2: 1 x 68 KB and 17 x 4 KB copies per tile are within noise
-      if (chunks < 1 || 69632 % chunks != 0 || (69632 / chunks) % 16 != 0) chunks = 1;
-      const char* f = getenv("CUTIE_B200_IMG_PREFETCH");
-      prefetch = f ? atoi(f) : 0;      // ... and so is an explicit L2 prefetch two tiles ahead
-      if (prefetch < 0 || prefetch > 64) prefetch = 0;
-    }
-    fp.img_chunks = chunks;
-    fp.img_prefetch = prefetch;
-    long long cum = 0;
-    for (int s = 0; s < base.segs.nseg; ++s) {
-      const long long n = base.segs.begin[s + 1] - base.segs.begin[s];
-      fp.img[s] = ia.img[s];
-      fp.img_bs[s] = ia.bs[s];
-      fp.img_tile0[s] = ia.phys[s] / 128;
-      fp.img_lo0[s] = (int)(ia.phys[s] % 128);
-      fp.img_tcum[s] = cum;
-      cum += n > 0 ? (fp.img_lo0[s] + n + 127) / 128 : 0;
-    }
-    for (int s = base.segs.nseg; s <= kMaxSeg; ++s) fp.img_tcum[s] = cum;
-    fp.nsplit = tc_split_count(B, base.Q, cum * 128);
-    fp.tiles_per_split = (int)((cum + fp.nsplit - 1) / fp.nsplit);
-    ++g_image_level_launches;
-  }
-  cudaError_t e = cudaMemsetAsync(ws + wl.count, 0, (size_t)(wl.emax0 - wl.count), st);   // count + dmax
-  if (e != cudaSuccess) return set_cuda_error("cudaMemsetAsync", e);
-  return launch_tc_filter(fp, B, st);
-}
 
 // FP16 plan over the key operand image: tile-sampled threshold pass -> k-th smallest slot minimum -> candidate filter
 // over the whole image -> exact re-rank.  Two memsets + four launches per call, whatever the bank size.
@@ -599,7 +508,7 @@ static int run_filtered_f16(const ScanParams& base, long long B, char* ws, const
   for (int s = base.segs.nseg; s <= kMaxSeg; ++s) fp.img_tcum[s] = cum;
   const int grid_x = f16_schedule(fp, B);
   const int groups = (fp.full_groups > 0 ? fp.splits_full : fp.splits_half) * 2 * F16_SLOTS;    // threshold slots per query
-  if (groups > TC_CAP_BIG) return fail(-1, "%s: too many key splits for the threshold workspace", "run_filtered_f16");
+  if (groups > CAND_CAP) return fail(-1, "%s: too many key splits for the threshold workspace", "run_filtered_f16");
   // sample every `stride`-th tile: every split of a query group should still see >= 8 tiles (its 64 slots then hold
   // minima over >= 16 tokens each); small banks are sampled whole
   const long long max_splits = fp.full_groups > 0 ? fp.splits_full : fp.splits_half;
@@ -608,7 +517,7 @@ static int run_filtered_f16(const ScanParams& base, long long B, char* ws, const
   if (stride < 1) stride = 1;
   const int ph = phase_begin(st);
   float* group_min = (float*)(ws + wl.cand_e);
-  float* emax = (float*)(ws + wl.emax0);
+  float* emax = (float*)(ws + wl.emax);
   cudaError_t e = cudaMemsetAsync(group_min, 0x7f, (size_t)B * base.Q * groups * 4, st);      // 0x7f7f7f7f = 3.4e38: "empty slot"
   if (e != cudaSuccess) return set_cuda_error("cudaMemsetAsync", e);
   fp.tile_stride = (int)stride;
@@ -639,7 +548,7 @@ static int run_filtered_f16(const ScanParams& base, long long B, char* ws, const
   fp.emax_in = emax;
   fp.cand_idx = (int*)(ws + wl.cand_idx);
   fp.count = (int*)(ws + wl.count);
-  fp.cap = TC_CAP_BIG;
+  fp.cap = CAND_CAP;
   rc = launch_f16_filter(fp, B, grid_x, false, st);
   if (rc) return rc;
   ++g_image_level_launches;
@@ -653,7 +562,7 @@ static int run_filtered_f16(const ScanParams& base, long long B, char* ws, const
   rp.n_total = base.n_total;
   rp.cand_idx = (const int*)(ws + wl.cand_idx);
   rp.count = (const int*)(ws + wl.count);
-  rp.cap = TC_CAP_BIG;
+  rp.cap = CAND_CAP;
   rp.top_k = base.top_k;
   rp.kpad = base.kpad;
   rp.out_idx = out_idx;
@@ -661,53 +570,6 @@ static int run_filtered_f16(const ScanParams& base, long long B, char* ws, const
   rp.out_sim = out_sim;
   rp.usage_acc = usage_acc;
   rc = launch_rerank(rp, B, st);
-  phase_mark(ph, st);
-  return rc;
-}
-
-static int run_filtered(const ScanParams& base, long long B, const Plan& pl, char* ws, const WsLayout& wl,
-                        int* out_idx, float* out_w, float* out_sim, unsigned long long* usage_acc,
-                        float* dbg_energy, const ImageArgs& ia, cudaStream_t st) {
-  float* emax[2] = {(float*)(ws + wl.emax0), (float*)(ws + wl.emax1)};
-  const float* emax_in = nullptr;
-  const int ph = phase_begin(st);
-  for (int l = 0; l < pl.levels; ++l) {
-    const bool last = (l == pl.levels - 1);
-    int rc = run_filter_level(base, B, pl.stride[l], emax_in, ws, wl, last ? dbg_energy : nullptr, ia, st);
-    if (rc) return rc;
-    phase_mark(ph, st);
-    if (!last) {
-      SelectParams sp;
-      sp.Q = base.Q;
-      sp.cand_e = (const float*)(ws + wl.cand_e);
-      sp.count = (const int*)(ws + wl.count);
-      sp.dmax = (const float*)(ws + wl.dmax);
-      sp.cap = TC_CAP_BIG;
-      sp.top_k = base.top_k;
-      sp.emax_out = emax[l & 1];
-      rc = launch_level_select(sp, B, base.kpad, st);
-      if (rc) return rc;
-      phase_mark(ph, st);
-      emax_in = emax[l & 1];
-    }
-  }
-  RerankParams rp;
-  memset(&rp, 0, sizeof(rp));
-  rp.segs = base.segs;
-  rp.qk = base.qk;
-  rp.qe = base.qe;
-  rp.Q = base.Q;
-  rp.n_total = base.n_total;
-  rp.cand_idx = (const int*)(ws + wl.cand_idx);
-  rp.count = (const int*)(ws + wl.count);
-  rp.cap = TC_CAP_BIG;
-  rp.top_k = base.top_k;
-  rp.kpad = base.kpad;
-  rp.out_idx = out_idx;
-  rp.out_w = out_w;
-  rp.out_sim = out_sim;
-  rp.usage_acc = usage_acc;
-  const int rc = launch_rerank(rp, B, st);
   phase_mark(ph, st);
   return rc;
 }
@@ -723,12 +585,11 @@ extern "C" size_t cutie_affinity_workspace_bytes(int64_t B, int64_t Q, int64_t n
   return ws_layout(B, Q, n_total, top_k).total;
 }
 
-// Banks with fewer tokens than this use the exact scan only (default 8192; env CUTIE_B200_TC_MIN /
-// CUTIE_B200_NO_TC=1).  Negative restores the default.  Process-wide; meant for tests and tuning.
+// Banks with fewer tokens than this use the exact scan only (default 6144).  Negative restores the default.
+// Process-wide; meant for tests and tuning.
 extern "C" void cutie_set_tc_min_tokens(int64_t n) { g_tc_min_override = n; }
 
-// Which plan cutie_affinity_topk will use: 1 = exact scan only, 2/3 = tcgen05 filter levels (see make_plan).
-// Per-phase device times (ms) of a filtered cutie_affinity_topk call: filter level, threshold select, ..., re-rank.
+// Per-phase device times (ms) of a filtered cutie_affinity_topk call: sample pass, threshold select, filter pass, re-rank.
 // cutie_debug_phase_timing(1) starts recording (a ring of the last 64 calls); cutie_debug_phase_times(calls_ago, ...)
 // waits for that call's last event and returns the number of phases written.
 extern "C" void cutie_debug_phase_timing(int enable) { g_phase_on = enable != 0; }
@@ -744,14 +605,15 @@ extern "C" int cutie_debug_phase_times(int64_t calls_ago, float* out_ms, int max
   return k;
 }
 
-// How many filter levels have been served from a key image so far in this process (diagnostics / tests).
+// How many filter passes have been served from a key image so far in this process (diagnostics / tests).
 extern "C" int64_t cutie_debug_image_level_launches(void) { return g_image_level_launches; }
 
-extern "C" int cutie_affinity_plan_levels(int64_t n_total, int top_k) { return make_plan(n_total, top_k).levels; }
+// Which plan cutie_affinity_topk_img will use when every segment has a key image: 0 = exact scan, 1 = FP16 filter.
+extern "C" int cutie_affinity_plan(int64_t n_total, int top_k) { return filter_plan(n_total, top_k) ? 1 : 0; }
 
 // Diagnostics: byte offset of the per-query candidate counters [B][Q] int32 inside the workspace (-1: exact-scan plan).
 extern "C" int64_t cutie_debug_ws_count_offset(int64_t B, int64_t Q, int64_t n_total, int top_k) {
-  if (make_plan(n_total, top_k).levels == 0) return -1;
+  if (!filter_plan(n_total, top_k)) return -1;
   return (int64_t)ws_layout(B, Q, n_total, top_k).count;
 }
 
@@ -779,9 +641,6 @@ static int fill_scan_params(ScanParams& sp, int num_segments, const void* const*
   sp.n_total = n_total;
   sp.top_k = top_k;
   sp.kpad = kpad;
-  sp.samp_begin = 0;
-  sp.samp_stride = 1;
-  sp.samp_count = n_total;
   return 0;
 }
 
@@ -809,31 +668,27 @@ extern "C" int cutie_affinity_topk_img(int num_segments, const void* const* seg_
   CUTIE_REQUIRE(workspace_bytes >= wl.total, "workspace too small");
   char* ws = (char*)workspace;
   cudaStream_t st = (cudaStream_t)stream;
-  const Plan pl = make_plan(n_total, top_k);
-  if (pl.levels == 0) {
-    const int ns0 = pick_splits(B, Q, n_total);
-    sp.part_val = (float*)(ws + wl.part);
-    sp.part_idx = (int*)(ws + wl.part + (size_t)B * ns0 * Q * kpad * 4);
-    return run_exact(sp, B, ns0, out_idx, out_w, out_sim, usage_acc, st);
-  }
-  ImageArgs ia;
-  memset(&ia, 0, sizeof(ia));
-  if (seg_key_image) {
+  if (filter_plan(n_total, top_k) && seg_key_image) {
     CUTIE_REQUIRE(seg_image_bstride && seg_phys_begin, "image strides / physical offsets missing");
-    ia.on = true;
+    ImageArgs ia;
+    memset(&ia, 0, sizeof(ia));
     ia.mu = key_mu;
     ia.seed_idx = seed_idx;
+    bool all_images = true;
     for (int s = 0; s < num_segments; ++s) {
-      if (seg_len[s] > 0 && !seg_key_image[s]) ia.on = false;          // a segment without an image: convert on the fly
+      if (seg_len[s] > 0 && !seg_key_image[s]) all_images = false;     // a segment without an image: exact scan
       CUTIE_REQUIRE(seg_phys_begin[s] >= 0, "negative physical offset");
       CUTIE_REQUIRE(((uintptr_t)seg_key_image[s] & 15) == 0, "key image must be 16-byte aligned");
       ia.img[s] = (const float*)seg_key_image[s];
       ia.bs[s] = seg_image_bstride[s];
       ia.phys[s] = seg_phys_begin[s];
     }
+    if (all_images) return run_filtered_f16(sp, B, ws, wl, out_idx, out_w, out_sim, usage_acc, ia, st);
   }
-  if (ia.on) return run_filtered_f16(sp, B, ws, wl, out_idx, out_w, out_sim, usage_acc, ia, st);
-  return run_filtered(sp, B, pl, ws, wl, out_idx, out_w, out_sim, usage_acc, nullptr, ia, st);
+  const int ns0 = pick_splits(B, Q, n_total);
+  sp.part_val = (float*)(ws + wl.part);
+  sp.part_idx = (int*)(ws + wl.part + (size_t)B * ns0 * Q * kpad * 4);
+  return run_exact(sp, B, ns0, out_idx, out_w, out_sim, usage_acc, st);
 }
 
 extern "C" int cutie_affinity_topk(int num_segments, const void* const* seg_key, const void* const* seg_shrinkage,
@@ -846,41 +701,6 @@ extern "C" int cutie_affinity_topk(int num_segments, const void* const* seg_key,
                                  nullptr, nullptr, nullptr, nullptr, nullptr, qk, qe, B, CK, Q, top_k, kpad, out_idx, out_w,
                                  out_sim,
                                  usage_acc, n_total, workspace, workspace_bytes, stream);
-}
-
-// Test hook: TF32 energies E[b,q,n] = -8 S of the tcgen05 filter for the whole bank (single level, no
-// threshold; n_total <= 4096 so that every token fits the candidate list).  dbg_energy [B, Q, n_total] floats.
-extern "C" int cutie_debug_tc_energy(int num_segments, const void* const* seg_key, const void* const* seg_shrinkage,
-                                     const int64_t* seg_len, const int64_t* seg_key_bstride,
-                                     const int64_t* seg_shr_bstride, const float* qk, const float* qe, int64_t B,
-                                     int64_t Q, int64_t n_total, float* dbg_energy, void* workspace,
-                                     size_t workspace_bytes, void* stream) {
-  CUTIE_REQUIRE(num_segments >= 1 && num_segments <= kMaxSeg && dbg_energy && workspace, "bad argument");
-  CUTIE_REQUIRE(n_total <= TC_CAP, "debug hook handles at most 4096 tokens");
-  ScanParams sp;
-  int rc = fill_scan_params(sp, num_segments, seg_key, seg_shrinkage, seg_len, seg_key_bstride, seg_shr_bstride, qk,
-                            qe, Q, 1, 32, n_total);
-  if (rc) return rc;
-  WsLayout wl;
-  memset(&wl, 0, sizeof(wl));
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-  wl.cand_idx = take((size_t)B * Q * TC_CAP_BIG * 4);
-  wl.cand_e = take((size_t)B * Q * TC_CAP_BIG * 4);
-  wl.count = take((size_t)B * Q * 4);
-  wl.dmax = take((size_t)B * Q * 4);
-  wl.emax0 = take((size_t)B * Q * 4);
-  wl.emax1 = take((size_t)B * Q * 4);
-  const size_t o_idx = take((size_t)B * Q * 32 * 4), o_w = take((size_t)B * Q * 32 * 4);
-  CUTIE_REQUIRE(workspace_bytes >= off, "workspace too small");
-  Plan pl;
-  pl.levels = 1;
-  pl.stride[0] = 1;
-  char* ws = (char*)workspace;
-  ImageArgs ia;
-  memset(&ia, 0, sizeof(ia));
-  return run_filtered(sp, B, pl, ws, wl, (int*)(ws + o_idx), (float*)(ws + o_w), nullptr, nullptr, dbg_energy, ia,
-                      (cudaStream_t)stream);
 }
 
 extern "C" int cutie_topk_merge(const float* part_val, const int32_t* part_idx, int64_t B, int64_t nparts, int64_t Q,

@@ -12,7 +12,7 @@
 //   filter pass  (sign +1): D = E_f16 - eps (P_n + R_n v_q)^2 - abs  <=  E_exact        -> candidate iff D < Emax_q
 //   sample pass  (sign -1): U = E_f16 + eps (P_n + R_n v_q)^2 + abs  >=  E_exact        -> threshold seeding
 // so a true top-k member is never dropped; survivors are re-ranked with the exact fp32 direct form
-// (affinity_rerank_kernel, affinity_tc.cu), which makes the final selection and weights bit-identical to the exact scan.
+// (affinity_rerank_kernel, below), which makes the final selection and weights bit-identical to the exact scan.
 //
 // Threshold seeding without a select over a token list: the sample pass walks every `stride`-th tile of the image and
 // every epilogue thread (= one query x one 64-column group of one CTA) keeps 32 running minima of U, one per register
@@ -391,6 +391,114 @@ __global__ void __launch_bounds__(256) f16_threshold_kernel(const F16ThresholdPa
   if (lane == 0) p.emax_out[bq] = emax;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Exact re-rank of the filter pass's candidates: one CTA (4 warps) per query.  Each warp evaluates chunks of 32
+// candidates with the exact fp32 direct form and keeps a sorted top-k; warp 0 merges and finalises (softmax,
+// usage).  A query whose candidate list overflowed is rescanned exhaustively (slow, correct, rare).
+//
+// Candidate key rows (256 B each) are fetched COALESCED -- a half-warp per row, 16 independent LDG.128 per lane in flight
+// -- and staged in shared memory; each lane then evaluates its own candidate from shared memory with the same
+// channel-sequential fp32 arithmetic as the exact scan (`exact_similarity_smem`), so results stay bit-identical.  (A lane
+// reading its own row straight from global memory touches 32 different 128-byte lines per instruction: 512 L1 wavefronts
+// per 32 candidates against 64 here, and the re-rank was bound by exactly that.)
+constexpr int RR_LD = 68;                 // floats per staged row: 272 B, 16-byte aligned, conflict-free LDS.128 per quarter-warp
+
+__device__ __forceinline__ float exact_similarity_smem(const float* __restrict__ krow, float shr, const float* __restrict__ a,
+                                                       const float* __restrict__ b) {
+  float acc = 0.f;
+#pragma unroll
+  for (int c4 = 0; c4 < CKD / 4; ++c4) {
+    const float4 kf = *reinterpret_cast<const float4*>(krow + 4 * c4);
+    float d;
+    d = fmaf(a[4 * c4 + 0], kf.x, -b[4 * c4 + 0]); acc = fmaf(d, d, acc);
+    d = fmaf(a[4 * c4 + 1], kf.y, -b[4 * c4 + 1]); acc = fmaf(d, d, acc);
+    d = fmaf(a[4 * c4 + 2], kf.z, -b[4 * c4 + 2]); acc = fmaf(d, d, acc);
+    d = fmaf(a[4 * c4 + 3], kf.w, -b[4 * c4 + 3]); acc = fmaf(d, d, acc);
+  }
+  return acc * (-shr * rsqrtf((float)CKD));
+}
+
+template <int NS>
+__global__ void __launch_bounds__(128) affinity_rerank_kernel(const RerankParams p) {
+  __shared__ float lv[4][KPAD_MAX];
+  __shared__ int li[4][KPAD_MAX];
+  __shared__ float qa[CKD], qb[CKD];
+  __shared__ __align__(16) float rows[4][32][RR_LD];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.y;
+  const long long q = blockIdx.x;
+  const long long bq = (long long)b * p.Q + q;
+  for (int u = 0; u < NS; ++u) { lv[warp][lane + 32 * u] = -CUDART_INF_F; li[warp][lane + 32 * u] = INT_MAX; }
+  if (tid < CKD) {
+    const long long off = ((long long)b * CKD + tid) * p.Q + q;
+    const float a = sqrtf(p.qe[off]);
+    qa[tid] = a;
+    qb[tid] = a * p.qk[off];
+  }
+  __syncthreads();
+  int n = p.count[bq];
+  const bool exhaustive = n > p.cap;
+  if (exhaustive) n = (int)p.n_total;
+  const int* cl = p.cand_idx + bq * p.cap;
+  const int h = lane >> 4, c4 = lane & 15;
+  for (int base = warp * 32; base < n; base += 128) {
+    const int j = base + lane;
+    int id = -1;
+    if (j < n) id = exhaustive ? j : cl[j];
+    const bool live = id >= 0;
+    float shr = 0.f;
+    const float* krow = nullptr;
+    if (live) {
+      const int sg = seg_of(p.segs.begin, p.segs.nseg, id);
+      const long long off = (long long)id - p.segs.begin[sg];
+      krow = p.segs.key[sg] + (long long)b * p.segs.key_bs[sg] + off * CKD;
+      shr = __ldg(p.segs.shr[sg] + (long long)b * p.segs.shr_bs[sg] + off);
+    }
+    // cooperative, coalesced fetch: at step it the two half-warps fetch rows 2 it and 2 it + 1 (16 lanes x 16 B each)
+    float4 piece[16];
+#pragma unroll
+    for (int it = 0; it < 16; ++it) {
+      const unsigned long long rp = __shfl_sync(0xffffffffu, (unsigned long long)krow, 2 * it + h);
+      piece[it] = rp ? __ldg(reinterpret_cast<const float4*>(rp) + c4) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+#pragma unroll
+    for (int it = 0; it < 16; ++it) *reinterpret_cast<float4*>(&rows[warp][2 * it + h][4 * c4]) = piece[it];
+    __syncwarp();
+    const float sv = live ? exact_similarity_smem(&rows[warp][lane][0], shr, qa, qb) : -CUDART_INF_F;
+    if (!live) id = INT_MAX;
+    const float kth = lv[warp][p.top_k - 1];
+    const int kthi = li[warp][p.top_k - 1];
+    unsigned bits = __ballot_sync(0xffffffffu, live && (sv > kth || (sv == kth && id < kthi)));
+    while (bits) {
+      const int src = __ffs(bits) - 1;
+      bits &= bits - 1;
+      const float cs = __shfl_sync(0xffffffffu, sv, src);
+      const int ci = __shfl_sync(0xffffffffu, id, src);
+      const float k2 = lv[warp][p.top_k - 1];
+      if (cs > k2 || (cs == k2 && ci < li[warp][p.top_k - 1]))
+        list_insert<NS>(&lv[warp][0], &li[warp][0], lane, p.top_k, cs, ci);
+    }
+    __syncwarp();      // the staging rows are overwritten by the next chunk
+  }
+  __syncthreads();
+  if (warp == 0) {
+    for (int w = 1; w < 4; ++w) {
+      for (int j = 0; j < p.top_k; ++j) {
+        const float cs = lv[w][j];
+        const int ci = li[w][j];
+        if (ci == INT_MAX) break;
+        const float k2 = lv[0][p.top_k - 1];
+        if (!(cs > k2 || (cs == k2 && ci < li[0][p.top_k - 1]))) break;     // sorted: the rest lose too
+        list_insert<NS>(&lv[0][0], &li[0][0], lane, p.top_k, cs, ci);
+      }
+    }
+    const long long oo = bq * p.kpad;
+    finalize_topk<NS>(&lv[0][0], &li[0][0], lane, p.top_k, p.kpad, p.out_idx + oo, p.out_w + oo,
+                      p.out_sim ? p.out_sim + oo : nullptr,
+                      p.usage_acc ? p.usage_acc + (long long)b * p.n_total : nullptr);
+  }
+}
+
 size_t f16_filter_smem_bytes() { return (size_t)(2 + F16_STAGES) * F16_OPER_BYTES + sizeof(F16Tail) + 64; }
 
 // CTA schedule for Q queries: returns the grid size; fills the group / split counts of `p`
@@ -435,6 +543,17 @@ int launch_f16_threshold(const F16ThresholdParams& p, long long B, cudaStream_t 
   f16_threshold_kernel<<<grid, 256, 0, st>>>(p);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return set_cuda_error("f16_threshold_kernel", e);
+  return 0;
+}
+
+int launch_rerank(const RerankParams& p, long long B, cudaStream_t st) {
+  dim3 grid((unsigned)p.Q, (unsigned)B);
+  if (p.kpad == 32)
+    affinity_rerank_kernel<1><<<grid, 128, 0, st>>>(p);
+  else
+    affinity_rerank_kernel<2><<<grid, 128, 0, st>>>(p);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return set_cuda_error("affinity_rerank_kernel", e);
   return 0;
 }
 

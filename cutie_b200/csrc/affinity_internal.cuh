@@ -1,47 +1,9 @@
-// Internal (non-ABI) interfaces between affinity.cu (exact scan, orchestration) and affinity_tc.cu
-// (tcgen05 candidate filter, level threshold hand-over, exact re-rank).
+// Internal (non-ABI) interfaces between affinity.cu (exact scan, orchestration) and affinity_f16.cu
+// (FP16 candidate filter over the key image, threshold select, exact re-rank).
 #pragma once
 #include "common.cuh"
 
 namespace cutie {
-
-// A "sample" of the bank: virtual indices i in [0, samp_count) map to tokens g = samp_begin + i * samp_stride
-// of the concatenated segments.  stride 1 = the whole bank.  Levels use nested samples (strides 256, 16, 1).
-
-struct TcFilterParams {
-  KeySegments segs;
-  const float* qk;
-  const float* qe;
-  long long Q;
-  long long samp_begin, samp_stride, samp_count;
-  int tiles_per_split, nsplit;
-  const float* emax_in;    // [B][Q] upper bound of the k-th smallest exact energy of the previous level; null = +inf
-  int* cand_idx;           // [B][Q][cap] token indices (per-query list, filled with atomics)
-  float* cand_e;           // [B][Q][cap] their TF32 energies
-  int* count;              // [B][Q] number of candidates (may exceed cap = overflow); zeroed by the caller
-  float* dmax;             // [B][Q] largest error bound used (atomicMax on the bit pattern); zeroed by the caller
-  int cap;
-  float* dbg_energy;       // optional [B][Q][samp_count] tf32 energies (tests)
-  // Image path (stride-1 level only): per segment the precomputed operand image of the arena it lives in
-  // (cutie_bank_key_image), addressed by physical 128-token tile.
-  int use_img;
-  int img_chunks;                  // bulk copies per 68 KB tile (69632 / chunks must be a multiple of 16)
-  int img_prefetch;                // L2 prefetch distance in tiles (0 = off)
-  const float* img[kMaxSeg];
-  long long img_bs[kMaxSeg];       // batch stride (floats)
-  long long img_tile0[kMaxSeg];    // first physical tile of the segment
-  int img_lo0[kMaxSeg];            // row of the segment's first token inside that tile
-  long long img_tcum[kMaxSeg + 1]; // prefix sums of the segments' tile counts
-};
-
-struct SelectParams {
-  long long Q;
-  const float* cand_e;
-  const int* count;
-  const float* dmax;
-  int cap, top_k;
-  float* emax_out;         // [B][Q]
-};
 
 struct RerankParams {
   KeySegments segs;
@@ -100,10 +62,6 @@ struct F16ThresholdParams {
 };
 int launch_f16_threshold(const F16ThresholdParams& p, long long B, cudaStream_t st);
 
-size_t tc_filter_smem_bytes();
-int tc_split_count(long long B, long long Q, long long samp_count);
-int launch_tc_filter(const TcFilterParams& p, long long B, cudaStream_t st);
-int launch_level_select(const SelectParams& p, long long B, int kpad, cudaStream_t st);
 int launch_rerank(const RerankParams& p, long long B, cudaStream_t st);
 
 }  // namespace cutie

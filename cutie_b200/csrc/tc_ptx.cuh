@@ -1,5 +1,5 @@
 // Inline-PTX helpers for the tcgen05 / mbarrier / bulk-copy kernels (sm_100a): shared by the affinity filter
-// (affinity_tc.cu, affinity_f16.cu) and the object-transformer attention kernels (qt_tc.cu).
+// (affinity_f16.cu) and the object-transformer attention kernels (qt_tc.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

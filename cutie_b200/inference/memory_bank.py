@@ -26,11 +26,6 @@ from cutie_b200 import kernels as K_
 from cutie_b200.kernels import BankSegment
 
 
-# The arenas keep a tcgen05 operand image of their keys (kernels.bank_key_image); False = the affinity filter
-# converts the fp32 rows inside the kernel instead (A/B switch for bench.py --no-key-image and tests).
-USE_KEY_IMAGE = True
-
-
 class TokenArena:
     """A set of same-length token-major arrays [B, capacity, C_i] with ring semantics."""
 
@@ -141,7 +136,7 @@ class TokenArena:
         """Bring the operand image up to date with every row written since the last call (new memory frames:
         one small launch; after a re-allocation or compaction: the whole arena).  `mu` [B, 64]: the bucket's key centre
         (the image holds k - mu); one image is only ever built with one centre."""
-        if not USE_KEY_IMAGE or 'key' not in self.arrays or self.widths.get('key') != 64:
+        if 'key' not in self.arrays or self.widths.get('key') != 64:
             return None
         if self.key_image is None:
             self.key_image = torch.zeros(self.B, K_.key_image_tiles(self.cap), K_.KEY_IMAGE_FLOATS,
@@ -328,8 +323,6 @@ class KeyValueMemoryStore:
         """The bucket's key centre: the mean key of the first tokens it ever served (the permanent first frame), fixed
         for the bucket's life.  Any vector is valid -- the energies do not depend on it -- it only tightens the FP16
         filter's error bound (network-derived keys sit on a large common mean)."""
-        if not USE_KEY_IMAGE:
-            return None
         mu = self.key_centres.get(bucket_id)
         if mu is None and regions:
             arena, runs = regions[0]

@@ -167,8 +167,7 @@ def affinity_topk(segments: Sequence[BankSegment], qk: torch.Tensor, qe: torch.T
         assert s.key.shape[2] == CK
     assert qk.is_contiguous() and qe.is_contiguous()
     PA, IA = ctypes.c_void_p * ns, ctypes.c_int64 * ns
-    _L = lib()
-    _lv = _L.cutie_affinity_plan_levels(_i64(n_total), ctypes.c_int(top_k))
+    plan = L.cutie_affinity_plan(_i64(n_total), ctypes.c_int(top_k))
     with_img = all(s.key_image is not None for s in segments)
     if with_img:
         for s in segments:
@@ -187,9 +186,9 @@ def affinity_topk(segments: Sequence[BankSegment], qk: torch.Tensor, qe: torch.T
                     IA(*[s.phys_begin for s in segments]), _ptr(mu), _ptr(seed_idx, torch.int32))
     else:
         img_args = (None, None, None, None, None)
-    # launches: exact scan = scan + merge; FP16 image plan = sample pass, threshold, filter pass, re-rank; TF32 levels
-    # (no image) = one filter per level, a select between levels, re-rank
-    with _call('affinity_topk', (4 if with_img else 2 * _lv) if _lv else 2):
+    # launches: exact scan (small banks, or no key images) = scan + merge; FP16 image plan = sample pass, threshold,
+    # filter pass, re-rank
+    with _call('affinity_topk', 4 if (plan and with_img) else 2):
         st = L.cutie_affinity_topk_img(
             ctypes.c_int(ns), PA(*[s.key.data_ptr() for s in segments]),
             PA(*[s.shrinkage.data_ptr() for s in segments]), IA(*[s.n for s in segments]),
@@ -223,7 +222,8 @@ def last_candidate_counts() -> Optional[torch.Tensor]:
 
 
 def set_tc_min_tokens(n: int):
-    """Banks with fewer tokens than n use the exact fp32 scan only; larger ones add the tcgen05 filter levels."""
+    """Banks with fewer tokens than n use the exact fp32 scan only; larger ones with key images take the FP16 filter
+    plan (default 6144; negative restores the default)."""
     lib().cutie_set_tc_min_tokens(_i64(n))
 
 
@@ -233,42 +233,23 @@ def phase_timing(enable: bool):
 
 
 def phase_times(calls_ago: int = 0):
-    """[ms per phase] of the affinity call `calls_ago` calls back: filter, select, filter, select, ..., re-rank."""
+    """[ms per phase] of the filtered affinity call `calls_ago` calls back: sample pass, threshold select, filter pass,
+    re-rank."""
     buf = (ctypes.c_float * 16)()
     n = lib().cutie_debug_phase_times(_i64(calls_ago), buf, ctypes.c_int(16))
     return [float(buf[i]) for i in range(n)]
 
 
 def image_level_launches() -> int:
-    """How many filter levels this process has served from a key image (bulk-copy producer) so far."""
+    """How many FP16 filter passes over a key image this process has run so far (one per filtered affinity call)."""
     f = lib().cutie_debug_image_level_launches
     f.restype = ctypes.c_int64
     return int(f())
 
 
-def affinity_plan_levels(n_total: int, top_k: int) -> int:
-    """0 = exact fp32 scan only; n >= 1 = n nested tcgen05 filter levels + exact re-rank of the survivors."""
-    return int(lib().cutie_affinity_plan_levels(_i64(n_total), ctypes.c_int(top_k)))
-
-
-def debug_tc_energy(segments: Sequence[BankSegment], qk: torch.Tensor, qe: torch.Tensor) -> torch.Tensor:
-    """Test hook: TF32 energies -8*S [B, Q, N] straight out of the tcgen05 filter."""
-    B, CK, Q = qk.shape
-    n_total = sum(s.n for s in segments)
-    out = torch.zeros(B, Q, n_total, dtype=torch.float32, device=qk.device)
-    ns = len(segments)
-    PA, IA = ctypes.c_void_p * ns, ctypes.c_int64 * ns
-    ws_bytes = B * Q * (16384 * 8 + 16 + 32 * 8) + (1 << 20)
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=qk.device)
-    with _call('debug_tc_energy', 2):
-        st = lib().cutie_debug_tc_energy(
-            ctypes.c_int(ns), PA(*[s.key.data_ptr() for s in segments]),
-            PA(*[s.shrinkage.data_ptr() for s in segments]), IA(*[s.n for s in segments]),
-            IA(*[s.key.stride(0) for s in segments]), IA(*[s.shrinkage.stride(0) for s in segments]),
-            _ptr(qk), _ptr(qe), _i64(B), _i64(Q), _i64(n_total), _ptr(out), _ptr(ws, torch.uint8),
-            ctypes.c_size_t(ws_bytes), _stream())
-    _check(st, 'cutie_debug_tc_energy')
-    return out
+def affinity_plan(n_total: int, top_k: int) -> int:
+    """0 = exact fp32 scan; 1 = FP16 filter over the key images + exact re-rank of the survivors (calls with images)."""
+    return int(lib().cutie_affinity_plan(_i64(n_total), ctypes.c_int(top_k)))
 
 
 def topk_merge(part_val: torch.Tensor, part_idx: torch.Tensor, top_k: int, n_total: int,

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define CUTIE_B200_ABI_VERSION 1
+#define CUTIE_B200_ABI_VERSION 2
 #define CUTIE_B200_MAX_SEGMENTS 4       /* long | permanent | ring piece a | ring piece b */
 #define CUTIE_B200_USAGE_FRAC_BITS 40   /* usage accumulators: uint64 fixed point, 2^-40 */
 
@@ -63,7 +63,7 @@ int cutie_affinity_topk(int num_segments, const void* const* seg_key, const void
  * 36 KB cp.async.bulk per tile), exact fp32 re-rank; the outputs are bit-identical to cutie_affinity_topk.
  * seed_idx ([B, Q, kpad] or NULL): per query top_k DISTINCT token indices (e.g. the previous frame's winners) whose
  * exact energies tighten the filter threshold; they never change the result, only how many candidates are re-ranked.
- * seg_key_image == NULL (or a NULL entry) = no images (TF32 levels with in-kernel producers). */
+ * seg_key_image == NULL (or a NULL entry for a non-empty segment) = no images: the exact fp32 scan, at every bank size. */
 int cutie_affinity_topk_img(int num_segments, const void* const* seg_key, const void* const* seg_shrinkage,
                             const int64_t* seg_len, const int64_t* seg_key_bstride, const int64_t* seg_shr_bstride,
                             const void* const* seg_key_image, const int64_t* seg_image_bstride,
@@ -73,27 +73,21 @@ int cutie_affinity_topk_img(int num_segments, const void* const* seg_key, const 
                             unsigned long long* usage_acc, int64_t n_total, void* workspace,
                             size_t workspace_bytes, void* stream);
 
-/* Execution plan of cutie_affinity_topk for a bank of n_total tokens: 0 = exact fp32 scan only; n >= 1 = n nested
- * tcgen05 (TF32) candidate-filter levels over strided samples (strides ..., 256, 16, 1) followed by an exact fp32
- * re-rank of the survivors.  All plans return the same selection and weights (a filter level only discards
- * tokens that provably cannot be in the top-k).
+/* Execution plan of cutie_affinity_topk_img for a bank of n_total tokens when every segment carries a key image:
+ * 0 = exact fp32 scan; 1 = the FP16 filter plan (csrc/affinity_f16.cu) followed by an exact fp32 re-rank of the
+ * survivors.  A call without images always runs plan 0.  Both plans return the same selection and weights (the
+ * filter only discards tokens that provably cannot be in the top-k).
  * cutie_set_tc_min_tokens: banks smaller than n use plan 0 (default 6144; negative restores the default). */
-int cutie_affinity_plan_levels(int64_t n_total, int top_k);
+int cutie_affinity_plan(int64_t n_total, int top_k);
 /* Diagnostics: byte offset of the per-query candidate counters inside the workspace of a filtered call (-1: exact scan). */
 int64_t cutie_debug_ws_count_offset(int64_t B, int64_t Q, int64_t n_total, int top_k);
 void cutie_set_tc_min_tokens(int64_t n);
-/* Diagnostics: per-phase device times (ms) of the filtered plan's launches (filter level, threshold select, ...,
- * exact re-rank) for one of the last 64 calls, measured in situ with events on the caller's stream. */
+/* Diagnostics: per-phase device times (ms) of the filtered plan's launches (sample pass, threshold select, filter
+ * pass, exact re-rank) for one of the last 64 calls, measured in situ with events on the caller's stream. */
 void cutie_debug_phase_timing(int enable);
 int cutie_debug_phase_times(int64_t calls_ago, float* out_ms, int max_phases);
-/* Number of filter levels served from a key image so far in this process (diagnostics / tests). */
+/* Number of filter passes served from a key image so far in this process (diagnostics / tests). */
 int64_t cutie_debug_image_level_launches(void);
-/* Test hook: raw TF32 energies E[b,q,n] = -8*S[n,q] computed by the tcgen05 filter over the whole bank
- * (dbg_energy [B,Q,n_total]); workspace >= cutie_affinity_workspace_bytes(B,Q,n_total,30) + B*Q*n_total*0. */
-int cutie_debug_tc_energy(int num_segments, const void* const* seg_key, const void* const* seg_shrinkage,
-                          const int64_t* seg_len, const int64_t* seg_key_bstride, const int64_t* seg_shr_bstride,
-                          const float* qk, const float* qe, int64_t B, int64_t Q, int64_t n_total,
-                          float* dbg_energy, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Merge `nparts` sorted candidate lists per query (part_val/part_idx [B, nparts, Q, kpad], unused slots
  * idx = INT32_MAX or -1 with val = -inf) into the global top_k + softmax; same outputs as cutie_affinity_topk.
@@ -215,10 +209,10 @@ int cutie_prob_to_mask(const float* prob, int64_t plane_stride, int64_t row_stri
  * Replaces the flatten + torch.cat growth of KeyValueMemoryStore.add (kv_memory_store.py:6-16,:136-149). */
 int cutie_bank_append(const float* src, int64_t src_bstride, float* dst_rows, int64_t dst_bstride, int64_t B,
                       int64_t C, int64_t n, void* stream);
-/* Build / refresh the tcgen05 operand image for tokens [phys_begin, phys_begin + n) of an arena (key_arena
+/* Build / refresh the FP16 tcgen05 operand image for tokens [phys_begin, phys_begin + n) of an arena (key_arena
  * [B, cap, 64], shr_arena [B, cap] token-major; image [B, image_tiles, 9216] floats, image_tiles*128 >= cap; key_mu [B, 64] or NULL: the image holds k - mu.
- * Tile t of the image holds tokens [128 t, 128 t + 128) as [shr k^2 | shr k | shr, 0, shr, -eps P^2, -2 eps P R,
- * -eps R^2, 0, 0] in the filter's shared-memory layout (4 SWIZZLE_128B K-blocks + tail; csrc/tc_operand.cuh).
+ * Tile t of the image holds tokens [128 t, 128 t + 128) as 36864 bytes of f16 operands [shr k^2 | shr k | error-bound
+ * tail] in the filter's shared-memory layout (2 SWIZZLE_128B K-blocks + tail; csrc/tc_operand_f16.cuh).
  * Called once per memory frame for the appended tokens -- the per-token part of get_similarity
  * (memory_utils.py:28-36: mk^2, shrinkage scaling) hoisted out of the per-frame read; no reference counterpart. */
 int cutie_bank_key_image(const float* key_arena, int64_t key_bstride, const float* shr_arena, int64_t shr_bstride,

@@ -14,7 +14,7 @@ def _declared():
     return sorted(set(re.findall(r'\b(cutie_[a-z0-9_]+)\s*\(', src)))
 
 
-def test_library_builds_loads_and_exports_header_symbols():
+def test_abi_v2_library_builds_loads_and_exports_header_symbols():
     import __graft_entry__ as ge
     ge.build()
     lib = ctypes.CDLL(ge.LIB)
@@ -22,7 +22,7 @@ def test_library_builds_loads_and_exports_header_symbols():
     assert len(names) >= 18
     for n in names:
         assert hasattr(lib, n), f'{n} declared in include/cutie_b200.h but not exported'
-    assert lib.cutie_b200_abi_version() == 1
+    assert lib.cutie_b200_abi_version() == 2
     lib.cutie_b200_last_error.restype = ctypes.c_char_p
     assert lib.cutie_b200_last_error() is not None
 
@@ -95,21 +95,20 @@ def test_sass_is_sm100a():
     assert 'sm_100a' in out
 
 
-def test_affinity_plan_is_pure_host_logic():
-    """Which passes cutie_affinity_topk runs for a bank size (no GPU needed): exact scan below the threshold,
-    nested tcgen05 filter levels (strides 16^l) above it, coarsest sample never above 4096 tokens."""
+def test_affinity_plan_rule_is_pure_host_logic():
+    """Which plan cutie_affinity_topk_img runs for a bank size (no GPU needed): exact scan below the threshold or when
+    the bank has fewer than 2k tokens, the FP16 image filter at and above it."""
     import __graft_entry__ as ge
     ge.build()
     lib = ctypes.CDLL(ge.LIB)
-    plan = lambda n, k=30: lib.cutie_affinity_plan_levels(ctypes.c_int64(n), k)
+    plan = lambda n, k=30: lib.cutie_affinity_plan(ctypes.c_int64(n), k)
     lib.cutie_set_tc_min_tokens(ctypes.c_int64(-1))
-    assert plan(100) == 0 and plan(1620) == 0 and plan(4860) == 0
-    assert plan(8100) == 2            # 8100/16 = 507-token all-pass sample, then the whole bank
-    assert plan(65536) == 2           # 4096-token sample
-    assert plan(65537) == 3 and plan(413100) == 3 and plan(414720) == 3
-    assert plan(20_000_000) == 5       # strides 65536, 4096, 256, 16, 1
+    assert plan(100) == 0 and plan(1620) == 0 and plan(4860) == 0 and plan(6143) == 0
+    assert plan(6144) == 1 and plan(8100) == 1 and plan(65537) == 1 and plan(413100) == 1 and plan(20_000_000) == 1
     lib.cutie_set_tc_min_tokens(ctypes.c_int64(256))
-    assert plan(333) == 1 and plan(59) == 0 and plan(4099) == 2
+    assert plan(333) == 1 and plan(256) == 1 and plan(255) == 0 and plan(4099) == 1
+    assert plan(59) == 0 and plan(300, 151) == 0 and plan(300, 150) == 1      # fewer than 2k tokens: exact scan
     lib.cutie_set_tc_min_tokens(ctypes.c_int64(1 << 40))
     assert plan(413100) == 0
     lib.cutie_set_tc_min_tokens(ctypes.c_int64(-1))
+    assert plan(413100) == 1

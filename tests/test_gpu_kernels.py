@@ -39,7 +39,8 @@ def make_bank(B, N, K, CK=64, CV=256, seed=0, cuts=()):
 
 
 def segments_of(K_, key, shr, vals, cuts):
-    """Split [B,N,..] tensors into physically separate (non-adjacent) runs like the arena does."""
+    """Split [B,N,..] tensors into physically separate (non-adjacent) runs like the arena does, each with the FP16 key
+    image of its own buffer (so banks at or above the filter threshold take the image plan)."""
     segs, lo = [], 0
     for hi in list(cuts) + [key.shape[1]]:
         # embed each run in a larger buffer so batch strides differ from n*C
@@ -53,7 +54,9 @@ def segments_of(K_, key, shr, vals, cuts):
             t = torch.zeros(v.shape[0], hi - lo + pad, v.shape[2]).cuda()
             t[:, :hi - lo] = v[:, lo:hi].cuda()
             vb.append(t[:, :hi - lo])
-        segs.append(K_.BankSegment(kb[:, :hi - lo], sb[:, :hi - lo], tuple(vb)))
+        img = torch.zeros(key.shape[0], K_.key_image_tiles(hi - lo + pad), K_.KEY_IMAGE_FLOATS).cuda()
+        K_.bank_key_image(kb, sb, 0, hi - lo, img)
+        segs.append(K_.BankSegment(kb[:, :hi - lo], sb[:, :hi - lo], tuple(vb), img, 0))
         lo = hi
     return segs
 

@@ -1,10 +1,10 @@
-"""tcgen05 candidate filters (TF32 with in-kernel producers; FP16 over the bank's key operand image) + exact re-rank:
-numerics of the tensor-core contraction itself, and bit-identity of the filtered paths with the exact fp32 scan."""
+"""tcgen05 FP16 candidate filter over the bank's key operand image + exact re-rank: the image layout, and bit-identity of
+the filtered path with the exact fp32 scan."""
 import pytest
 import torch
 
 from oracle import memory_math as mm
-from tests.test_gpu_kernels import K_, check_topk, make_bank, segments_of  # noqa: F401
+from tests.test_gpu_kernels import K_, check_topk, segments_of  # noqa: F401
 
 pytestmark = pytest.mark.gpu
 
@@ -16,47 +16,27 @@ def tc_everywhere(K_):
     K_.set_tc_min_tokens(-1)
 
 
-@pytest.mark.parametrize('B,N,Q,cuts,scale', [(1, 128, 128, (), 1.0), (2, 300, 200, (77,), 1.0), (1, 1000, 130, (128, 500, 501), 3.0)])
-def test_tf32_energy_matches_exact_within_bound(K_, B, N, Q, cuts, scale):
-    key, shr, vals = make_bank(B, N, 0, seed=4)
-    key = key * scale
-    g = torch.Generator().manual_seed(9)
-    qk = torch.randn(B, 64, Q, generator=g) * scale
-    qe = torch.sigmoid(torch.randn(B, 64, Q, generator=g))
-    segs = segments_of(K_, key, shr, vals, cuts)
-    d = K_.debug_tc_energy(segs, qk.cuda(), qe.cuda()).cpu().double()                 # [B,Q,N]
-    truth = -8.0 * mm.similarity_direct(key.transpose(1, 2), shr.unsqueeze(1), qk, qe).transpose(1, 2)   # [B,Q,N]
-    # The MMA output folds the rigorous per-(token, query) error bound in:  d = E_tf32 - eps*shr_n*(|k_n| + sqrt(b2_q))^2
-    # so it must be a LOWER bound of the exact energy, and never further than 2*eps*(...) below it.
-    knorm = key.double().norm(dim=2)                                                   # [B,N]
-    vq = (qe.double() * qk.double() ** 2).sum(1).sqrt()                                # [B,Q]
-    s2 = shr.double()[:, None, :] * (knorm[:, None, :] + vq[:, :, None]) ** 2
-    assert (d <= truth + 1e-9).all(), f'filter value above the exact energy by {float((d - truth).max()):.3e}'
-    assert (truth - d <= 2.0 * 1.66e-3 * s2).all(), f'max slack ratio {float(((truth - d) / (1.65e-3 * s2)).max()):.3f}'
-    # the TF32 contraction itself (bound removed) is far more accurate than its worst case
-    e_tf32 = d + 1.65e-3 * s2
-    assert float(((e_tf32 - truth).abs() / truth.abs().clamp_min(1e-6)).median()) < 1e-3
-
-
 @pytest.mark.parametrize('B,N,Q,K,top_k,cuts', [
-    (1, 333, 77, 2, 30, ()),                   # single level: every token is a candidate
+    (1, 333, 77, 2, 30, ()),                   # three image tiles
     (2, 1000, 130, 2, 30, (128, 500, 501)),    # four segments, batch 2
     (1, 4099, 1620, 3, 30, (4000,)),           # 480p query count
     (1, 5000, 300, 1, 64, (100,)),             # kpad 64
-    (1, 70001, 96, 1, 30, (1620, 30000)),      # 3 nested levels (strides 256 -> 16 -> 1)
+    (1, 70001, 96, 1, 30, (1620, 30000)),      # three segments
 ])
-def test_filtered_path_matches_oracle_and_exact_scan(K_, tc_everywhere, B, N, Q, K, top_k, cuts):
-    assert K_.affinity_plan_levels(N, top_k) >= 1
+def test_fp16_filter_matches_oracle_and_exact_scan(K_, tc_everywhere, B, N, Q, K, top_k, cuts):
+    assert K_.affinity_plan(N, top_k) == 1
+    before = K_.image_level_launches()
     idx_tc, w_tc = check_topk(K_, B, N, Q, K, top_k, cuts)          # all oracle assertions on the filtered path
+    assert K_.image_level_launches() == before + 1, 'the FP16 image plan did not run'
     K_.set_tc_min_tokens(1 << 40)                                   # same inputs through the exact scan only
-    assert K_.affinity_plan_levels(N, top_k) == 0
+    assert K_.affinity_plan(N, top_k) == 0
     idx_ex, w_ex = check_topk(K_, B, N, Q, K, top_k, cuts)
     assert torch.equal(idx_tc, idx_ex), 'filtered selection differs from the exact scan'
     assert torch.equal(w_tc, w_ex), 'weights are not bit-identical'
 
 
 def test_filter_keeps_duplicates_and_near_duplicates(K_, tc_everywhere):
-    """Near-duplicate frames (the hard case of SURVEY.md Appendix B): many tokens within TF32 noise of each other."""
+    """Near-duplicate frames (the hard case of SURVEY.md Appendix B): many tokens within FP16 noise of each other."""
     g = torch.Generator().manual_seed(2)
     base = torch.randn(1, 500, 64, generator=g) * 4
     key = torch.cat([base + 1e-3 * torch.randn(1, 500, 64, generator=g) for _ in range(8)], 1)   # 4000 tokens
@@ -65,14 +45,17 @@ def test_filter_keeps_duplicates_and_near_duplicates(K_, tc_everywhere):
     qk = base[:, :200].transpose(1, 2).contiguous() + 1e-3 * torch.randn(1, 64, 200, generator=g)
     qe = torch.sigmoid(torch.randn(1, 64, 200, generator=g))
     segs = segments_of(K_, key, shr, vals, (1500,))
+    assert K_.affinity_plan(4000, 30) == 1
+    before = K_.image_level_launches()
     idx, w, sim = K_.affinity_topk(segs, qk.cuda(), qe.cuda(), 30, want_sim=True)
+    assert K_.image_level_launches() == before + 1, 'the FP16 image plan did not run'
     K_.set_tc_min_tokens(1 << 40)
     idx2, w2, sim2 = K_.affinity_topk(segs, qk.cuda(), qe.cuda(), 30, want_sim=True)
     assert torch.equal(idx, idx2) and torch.equal(w, w2) and torch.equal(sim, sim2)
 
 
 # ---------------------------------------------------------------------------------------------------------
-# key image (bulk-copy producer of the stride-1 filter level)
+# key image layout and the image plan's edge cases
 # ---------------------------------------------------------------------------------------------------------
 def _image_offsets(row, elem):
     """Byte offset of FP16 operand element `elem` (0..143) of token row `row` inside a 36864-byte tile
@@ -158,14 +141,14 @@ def _arena_bank(K_, B, layout, seed, centred=False):
     (1, 300, 30, [(9000, 0, 9000)]),                                        # aligned, one arena
     (1, 260, 30, [(3000, 1, 2999), (20000, 12345, 7000), (20000, 0, 5001)]),    # ring wrap: tail run + head run
     (2, 130, 30, [(700, 130, 500), (8000, 127, 7000), (8000, 7999, 1), (6000, 128, 3000)]),   # 4 runs, batch 2
-    (1, 96, 64, [(80000, 3, 70001)]),                                       # 3 levels, kpad 64
+    (1, 96, 64, [(80000, 3, 70001)]),                                       # unaligned start, kpad 64
     (1, 1620, 30, [(420000, 1000, 413100)]),                                # BASELINE cfg 2 bank size
 ])
 @pytest.mark.parametrize('centred', [False, True])
-def test_image_path_is_bit_identical_to_exact_scan(K_, tc_everywhere, B, Q, top_k, layout, centred):
+def test_image_plan_is_bit_identical_to_exact_scan(K_, tc_everywhere, B, Q, top_k, layout, centred):
     segs, key, shr = _arena_bank(K_, B, layout, seed=11, centred=centred)
     N = key.shape[1]
-    assert K_.affinity_plan_levels(N, top_k) >= 2
+    assert K_.affinity_plan(N, top_k) == 1
     g = torch.Generator().manual_seed(5)
     qk = (torch.randn(B, 64, Q, generator=g) * 1.5).cuda() + (segs[0].key_mu[:, :, None] if centred else 0.0)
     qe = torch.sigmoid(torch.randn(B, 64, Q, generator=g)).cuda()
@@ -173,7 +156,7 @@ def test_image_path_is_bit_identical_to_exact_scan(K_, tc_everywhere, B, Q, top_
     acc = torch.zeros(B, N, dtype=torch.int64, device='cuda')
     idx, w, sim = K_.affinity_topk(segs, qk, qe, top_k, usage_acc=acc, want_sim=True)
     assert K_.image_level_launches() == before + 1, 'the FP16 image plan did not run'
-    plain = [K_.BankSegment(s.key, s.shrinkage, ()) for s in segs]          # same bank, in-kernel producers
+    plain = [K_.BankSegment(s.key, s.shrinkage, ()) for s in segs]          # same bank without images: exact scan
     idx_p, w_p, sim_p = K_.affinity_topk(plain, qk, qe, top_k, want_sim=True)
     assert K_.image_level_launches() == before + 1
     K_.set_tc_min_tokens(1 << 40)                                           # exact fp32 scan only
